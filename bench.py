@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the sylph_b200 hot paths (contract: see DESIGN.md §Measurement).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload sketch|profile]
+                  [--dump-outputs DIR]
 
 Primary line (default --workload sketch) = BASELINE.json configs[1]:
   sketch 1 Gbp of synthetic 150 bp single-end reads, k=31 c=200, per GPU (weak scaling: every
@@ -77,7 +78,44 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--fixed-warmup", action="store_true",
                     help="exactly --warmup untimed steps (no settle loop): for runs under ncu, whose numbers are never bench values")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what each timed path returned in its last step as DIR/<name>.npy "
+                         "(float64, at most 64 MiB in all), to compare two builds output for output")
     return ap.parse_args()
+
+
+# --dump-outputs: rows kept per table (a longer table is cut to a fixed, seeded sample of its rows).  In float64
+# columns that is at most 3 x 8 B x 2^20 (sketch) + 2 x 8 B x 2^20 (genome k-mers) + 2 x 8 B x 2^19 (tracked)
+# + 6 x 8 B x 2^16 (per genome) + 21 x 8 B x 2^14 (profile rows) = 53.6 MiB
+DUMP_ROWS = {"sketch": 1 << 20, "sketch_stats": 1, "genome_kmers": 1 << 20, "genome_tracked": 1 << 19, "genomes": 1 << 16,
+             "profile": 1 << 14}
+DUMP_MAX_BYTES = 64 << 20
+_dumped = [0]
+
+
+def dump_table(out_dir, name, cols):
+    """Write the equal-length columns `cols` (field -> array) of one output table as DIR/<name>_<field>.npy in float64,
+    and its row count as DIR/<name>_rows.npy.  uint64 fields are split into exact 32-bit halves <field>_hi / <field>_lo
+    (float64 holds 53 bits).  A table longer than DUMP_ROWS[name] keeps a seeded sample of rows: the same rows in
+    every run that produced as many."""
+    import numpy as np
+    n = len(next(iter(cols.values())))
+    idx = np.arange(n)
+    if n > DUMP_ROWS[name]:
+        idx = np.sort(np.random.default_rng(0x5EED).choice(n, DUMP_ROWS[name], replace=False))
+    out = {"rows": np.array([n], dtype=np.float64)}
+    for field, a in cols.items():
+        a = np.asarray(a)[idx]
+        if a.dtype == np.uint64:
+            out[field + "_hi"], out[field + "_lo"] = a >> np.uint64(32), a & np.uint64(0xFFFFFFFF)
+        else:
+            out[field] = a
+    os.makedirs(out_dir, exist_ok=True)
+    for field, a in out.items():
+        a = a.astype(np.float64)
+        _dumped[0] += a.nbytes
+        assert _dumped[0] <= DUMP_MAX_BYTES, "--dump-outputs exceeds 64 MiB"
+        np.save(os.path.join(out_dir, "%s_%s.npy" % (name, field)), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -339,9 +377,12 @@ def bench_sketch(args, ctx, rank, world, local):
     state = {}
 
     def step_resident():
+        # frees the previous step's sketch: every step frees one and makes one, and the last timed one stays readable
+        if "s" in state:
+            state["s"].free()
         s = ctx.sketch_sequences(bases, off, k=K, c=C)
         state["n"] = len(s)
-        s.free()
+        state["s"] = s
 
     # clocks are sampled from before the warm-up to the end of the timed region: nvidia-smi needs ~100 ms to
     # start and its first query can stall the GPU, so neither may fall inside the (tens of ms) timed region;
@@ -386,6 +427,13 @@ def bench_sketch(args, ctx, rank, world, local):
     ctx.enable_timing(False)
     total_bases = sum_over_ranks(float(n_bases), world)
     value = total_bases * args.steps / (ms * 1e-3)
+    s = state.pop("s")
+    if args.dump_outputs and rank == 0:
+        h, c = s.download()
+        dump_table(args.dump_outputs, "sketch", {"hash": h, "count": c})
+        dump_table(args.dump_outputs, "sketch_stats", {"num_dup_removed": [s.num_dup_removed],
+                                                       "mean_read_length": [s.mean_read_length]})
+    s.free()
 
     # one extra call for the survivor count (algorithmic output bytes of the seeding kernel)
     surv_buf = torch.empty(int(n_bases / C * 1.3 + 65536) * 2, dtype=torch.int64, device="cuda")
@@ -433,7 +481,7 @@ def bench_sketch(args, ctx, rank, world, local):
 
     for _ in range(max(1, args.warmup // 2)):
         step_e2e()
-    e2e_steps = max(1, min(args.steps, 10))
+    e2e_steps = args.steps
     e2e_state["t"] = []
     ctx.enable_timing(True)
     ctx.seed_kernel_time(reset=True)
@@ -491,31 +539,31 @@ def bench_genomes(args, ctx, rank, world, local):
     st = {}
 
     def step():
-        g = ctx.sketch_genomes(bases, off, goff, k=K, c=C)
-        st["g"] = g
+        # frees the previous step's sketches: every step frees one batch and makes one, and the last timed one stays
+        if "g" in st:
+            st["g"].free()
+        st["g"] = ctx.sketch_genomes(bases, off, goff, k=K, c=C)
 
     for _ in range(max(args.warmup, 3)):
         step()
-        st["g"].free()
     ctx.enable_timing(True)
     ctx.seed_kernel_time(reset=True)
     ctx.kernel_time("genome_post", reset=True)
     l0 = ctx.launches
-
-    def tstep():
-        step()
-        st["g"].free()
-
-    ms, _ = timed(tstep, args.steps, world)
+    ms, _ = timed(step, args.steps, world)
     launches = ctx.launches - l0
     kms = ctx.seed_kernel_time(reset=True)[0] / args.steps
     pms = ctx.kernel_time("genome_post", reset=True)[0] / args.steps
     ctx.enable_timing(False)
     n_bases = float(bases.numel())
     value = sum_over_ranks(n_bases, world) * args.steps / (ms * 1e-3)
-    step()
     g = st["g"]
     d = g.download()
+    if args.dump_outputs and rank == 0:
+        dump_table(args.dump_outputs, "genome_kmers", {"hash": d["kmers"]})
+        dump_table(args.dump_outputs, "genome_tracked", {"hash": d["tracked"]})
+        dump_table(args.dump_outputs, "genomes", {"kmer_end": d["kmer_off"][1:], "tracked_end": d["tracked_off"][1:],
+                                                  "gn_size": d["gn_size"]})
     peak, peak_src = measured_peak_hbm()
     n_surv_est = int(d["kmer_off"][-1] + d["tracked_off"][-1])
     alg = n_bases + 16.0 * n_surv_est   # SURVEY §8(d), positions variant: 1 B/base + 16 B per survivor
@@ -637,6 +685,8 @@ def bench_pairs(args, ctx, rank, world, local, reads):
     pairs = float(n_samples) * G_total
     value = pairs * args.steps / (ms * 1e-3)
     rows = st["rows"]
+    if args.dump_outputs and rank == 0:
+        dump_table(args.dump_outputs, "profile", {f: rows[f] for f in rows.dtype.names if f != "reserved"})
     out = {"metric": "(sample x genome) containment pairs/s", "value": value, "unit": "pairs/s", "ms_per_step": ms / args.steps,
            "wall_ms_per_step": wall / args.steps, "steps": args.steps, "gpu_launches": int(launches),
            "config": profile_config(args, world),

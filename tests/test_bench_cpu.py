@@ -44,6 +44,34 @@ def test_both_arms_share_the_config_object():
     assert bench.profile_config(A, 1)["samples"] == 1 and bench.profile_config(A, 8)["samples"] == 16
 
 
+def test_dump_table_is_exact_seeded_and_bounded(tmp_path):
+    """--dump-outputs' writer: float64 files only, uint64 values kept exactly (above 2^53), a table longer than its
+    row limit cut to the same seeded sample in every run, and the row count recorded."""
+    sys.path.insert(0, REPO)
+    import numpy as np
+    import bench
+    n = bench.DUMP_ROWS["sketch"] + 5000
+    i = np.arange(n, dtype=np.uint64)
+    h = np.uint64(1 << 63) | (i << np.uint64(33)) | np.uint64(0x2345_6789)   # the row index sits in bits 33..62
+    c = (i % np.uint64(7)).astype(np.uint32)
+    bench._dumped[0] = 0
+    for d in ("a", "b"):
+        bench.dump_table(str(tmp_path / d), "sketch", {"hash": h, "count": c})
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(os.listdir(tmp_path / "b")) == ["sketch_count.npy", "sketch_hash_hi.npy", "sketch_hash_lo.npy",
+                                                            "sketch_rows.npy"]
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float64 and np.array_equal(a, b), f
+    load = lambda f: np.load(tmp_path / "a" / ("sketch_%s.npy" % f))  # noqa: E731
+    got = (load("hash_hi").astype(np.uint64) << np.uint64(32)) | load("hash_lo").astype(np.uint64)
+    rows = (got >> np.uint64(33)) & np.uint64((1 << 30) - 1)
+    assert len(got) == bench.DUMP_ROWS["sketch"] and load("rows").tolist() == [n]
+    assert np.all(rows[1:] > rows[:-1]) and int(rows[-1]) < n              # distinct rows, in table order
+    assert np.array_equal(got, h[rows.astype(np.int64)]) and np.array_equal(load("count"), c[rows.astype(np.int64)])
+    bench._dumped[0] = 0
+
+
 def test_clock_sampler_degrades_without_a_gpu():
     sys.path.insert(0, REPO)
     import bench
